@@ -11,6 +11,10 @@ A "step" = one batched call that runs ALL GN iterations of ONE object list (BASE
 the solved (pose, code, loss, status) records go back to rank 0 INSIDE the step: stored by the solve kernel
 straight into rank 0's HBM over NVLink (CUDA-IPC peer mapping; `--exchange nccl` = all-gather instead).
 Prints ONE JSON line on rank 0.
+
+  --dump-outputs DIR   after the timed steps, rank 0 writes what the last timed step computed, as the arrays a caller
+                       of Optimizer.reconstruct_batch receives (DIR/<name>.npy, float32; NaN where that caller gets
+                       None).  The inputs are seeded: the same arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -22,6 +26,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing is written into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -59,7 +64,30 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=4, help="objects in the CPU baseline sample")
     ap.add_argument("--exchange", default="auto", choices=["auto", "peer", "nccl"],
                     help="multi-GPU result exchange: NVLink peer stores from the solve kernel (default) or NCCL all-gather")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
+
+
+def dump_outputs(out_dir, rec, code_len):
+    """(n, RESULT_FLOATS) solver records -> the per-object results a caller of reconstruct_batch receives, stacked."""
+    from dsp_slam_b200.distributed import records_to_results
+    res = records_to_results(rec, code_len)
+    nan = np.float32(np.nan)
+
+    def col(key, shape):
+        return np.stack([np.asarray(r[key], np.float32) if r.get(key) is not None else np.full(shape, nan) for r in res])
+    arrays = {"t_cam_obj": col("t_cam_obj", (4, 4)), "code": col("code", (code_len,)),
+              "is_good": col("is_good", ()), "loss": col("loss", ()), "status": col("status", ()),
+              "n_valid": col("n_valid", ()), "n_band": col("n_band", ())}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def make_inputs(workload, world=1):
@@ -191,7 +219,7 @@ def run_reference(args):
     if rank != 0:
         return
     B, M, nfg, nbg, cls, cfgname, sdf_only, desc = WORKLOADS[args.workload]
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     val, dt = cpu_baseline(args.workload, args.cpu_sample, steps=steps, warmup=min(args.warmup, 1))
     cores = os.cpu_count()
     out = {
@@ -301,6 +329,10 @@ def run_ours(args):
             time.sleep(0.02)
     ms_local, t0, t1 = timed_loop(step, args.steps)
     clocks = sampler.stop(t0, t1) if sampler else None
+    if args.dump_outputs:               # before anything else runs on the resident batch
+        rec = sh.gather_records() if sh else np.frombuffer(solver.results_raw(), np.float32).reshape(n_total, -1)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, rec, opt.code_len)
     launches_per_step = solver.counters()["kernel_launches"]
     ms = max_over_ranks(ms_local)
     value = n_total / (ms * 1e-3)
